@@ -7,7 +7,7 @@ multivariate TPE, default gamma (n_below = 25) -- SURVEY.md section 8d.  One *st
 suggestion = split + both Parzen-estimator builds + C candidate draws + log l(x) and log g(x) over
 the C x K x P grid + argmax.  Nothing is cached between steps.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 ``value``  device-resident throughput: the K timed steps go through the C ABI (tpe_suggest) with the
            history already in HBM; time = wall clock between device synchronisations around the K
@@ -30,6 +30,13 @@ the C x K x P grid + argmax.  Nothing is cached between steps.
 ``--impl reference``  the reference ITSELF on the host cores: optuna's own ``_split_trials``,
            ``_ParzenEstimator`` and ``log_pdf`` (oracle/_ref, unmodified) on the same 100k-trial study;
            each step is a bounded sample (see run_reference).
+``--dump-outputs DIR``  after the timed steps, rank 0 writes what the last timed step computed as float64 .npy files:
+           what tpe_suggest returns (x, acq, best) and the candidates behind it (tpe_get_candidates: candidates,
+           log_l, log_g; 1.1 MB in all).  The inputs are seeded, so two builds can be compared output for output.
+           log_g is a sum over 100k kernels whose order varies from run to run: on a B200 two runs of the same build
+           differ in its last bits (2.5e-15 relative); everything else is bit-identical.
+
+The benchmark writes nothing into the source tree (no bytecode caches either): it may run from a read-only checkout.
 """
 from __future__ import annotations
 
@@ -44,6 +51,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -169,9 +177,8 @@ NAMES = [f"x{j:02d}" for j in range(N_PARAMS)]
 
 
 def import_optuna():
-    """The reference package: an installed optuna, else the copy under oracle/_ref (oracle/build_ref.py)."""
-    from oracle import build_ref, ref
-    build_ref.build()
+    """The reference package: an installed optuna, else the copy build() left under oracle/_ref (oracle/build_ref.py)."""
+    from oracle import ref
     if not ref.enable():
         raise RuntimeError("optuna is not importable and oracle/_ref is absent (run `python oracle/build_ref.py`)")
     import optuna
@@ -314,6 +321,15 @@ def cpu_baseline_leg(optuna, study, space) -> dict:
 # -------------------------------------------------------------------------------------------------
 # GPU arm
 # -------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir: str, eng, x, acq, best) -> None:
+    """The last timed suggestion as DIR/<name>.npy (float64): the returned point, acquisition value and candidate
+    index, and the 4096 candidates with their log-densities under l(x) and g(x)."""
+    os.makedirs(out_dir, exist_ok=True)
+    smp, ll, lg = eng.get_candidates()
+    for name, a in (("x", x), ("acq", acq), ("best", best), ("candidates", smp), ("log_l", ll), ("log_g", lg)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_b200(args) -> None:
     import torch
     import torch.distributed as dist
@@ -383,7 +399,7 @@ def run_b200(args) -> None:
     launches = 0
     t0 = time.perf_counter()
     for i in range(args.warmup, total):
-        eng.suggest(cols, Unp[i], 1, **cfg)
+        x_last, acq_last, best_last = eng.suggest(cols, Unp[i], 1, **cfg)
         ms, nl = eng.last_timing()
         stage += ms
         launches += nl
@@ -391,6 +407,8 @@ def run_b200(args) -> None:
     t1 = time.perf_counter()
     barrier()
     clk = clocks.stop() if rank == 0 else {}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, x_last, acq_last, best_last)
     kernel_name = eng.last_logpdf_kernel()
     wall = t1 - t0
     dev_ms = float(stage[8])
@@ -799,6 +817,7 @@ def main() -> None:
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the univariate / batched / cold extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     ap.add_argument("--n-trials", type=int, default=N_TRIALS, help="development only: a shorter history (the line then "
                     "says so in config.n_trials); the benchmark is the default")
     args = ap.parse_args()

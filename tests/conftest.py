@@ -1,3 +1,4 @@
+import itertools
 import os
 import sys
 
@@ -59,7 +60,8 @@ def make_sampler(request, monkeypatch):
         return s
 
     def reference(ties=False, **kw):
-        """The sampler to compare with: the live reference -- except for the CUDA engine in univariate scenarios
+        """The sampler to compare with: the reference (run live only to store its results, see `yardstick`) -- except
+        for the CUDA engine in univariate scenarios
         with repeated numeric observations, where the reference's bandwidths depend on the tie order of numpy's
         UNSTABLE argsort (parzen_estimator.py:200; CPU-dispatch dependent) while the CUDA path sorts stably
         (DESIGN.md section 4): there the yardstick is the same host glue answered by the stable-sort oracle.
@@ -73,8 +75,20 @@ def make_sampler(request, monkeypatch):
         from optuna.samplers import TPESampler
         return TPESampler(**kw)
 
+    def yardstick(tag, scenario, ties=False, **kw):
+        """What the yardstick computed in `scenario(sampler) -> study`, as tests._reference_golden.stored_study: the
+        stored result of the reference (run `tag` of this test) -- or, where `reference` names the stable-sort
+        oracle, that oracle's run now."""
+        from tests._reference_golden import node_key, recorded, stored_study, summarize
+        if request.param == "cuda" and ties and not kw.get("multivariate", False):
+            return stored_study(summarize(scenario(reference(ties, **kw))))
+        return stored_study(recorded(f"{node_key(request.node.name)}/{tag}",
+                                     lambda: summarize(scenario(reference(**kw)))))
+
     make.kind = request.param
     make.reference = reference
+    make.yardstick = yardstick
+    make.runs = itertools.count()
     yield make
     for s in made:
         s.close()

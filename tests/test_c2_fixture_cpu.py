@@ -1,10 +1,10 @@
 """The full-size config-2 fixture (tests/golden/c2_logpdf.npz) is what the GPU test measures the grid kernels
-against: pin it -- a few of its points recomputed with the oracle (bit for bit) and with the live reference's own
-_ParzenEstimator.log_pdf on the same 100 000-kernel estimator (1e-12)."""
+against: pin it -- a few of its points recomputed with the oracle (bit for bit) and compared with the reference's own
+_ParzenEstimator.log_pdf on the same 100 000-kernel estimator (1e-12; stored by tests/_reference_golden.py)."""
 import numpy as np
-import pytest
 
 from oracle import tpe_oracle as orc
+from tests._reference_golden import recorded
 from tests._util import load
 
 
@@ -24,14 +24,19 @@ def test_fixture_points_against_oracle_and_live_reference():
     mb = orc.build_mixture(X[below], params, cfg)
     assert np.array_equal(orc.mixture_log_pdf(ma, x), g["logg"][pick])
     assert np.array_equal(orc.mixture_log_pdf(mb, x), g["logl"][pick])
-    optuna = pytest.importorskip("optuna")
-    from optuna.samplers._tpe.parzen_estimator import _ParzenEstimator, _ParzenEstimatorParameters
-    from optuna.samplers._tpe.sampler import default_weights
-    names = [f"x{j:02d}" for j in range(P)]
-    space = {n: optuna.distributions.FloatDistribution(0.0, 1.0) for n in names}
-    prm = _ParzenEstimatorParameters(prior_weight=1.0, consider_magic_clip=True, consider_endpoints=False,
-                                     weights=default_weights, multivariate=True, categorical_distance_func={})
-    pts = {n: x[:, j] for j, n in enumerate(names)}
-    for rows, want in ((above, g["logg"][pick]), (below, g["logl"][pick])):
-        pe = _ParzenEstimator({n: X[rows, j] for j, n in enumerate(names)}, space, prm)
-        np.testing.assert_allclose(pe.log_pdf(pts), want, rtol=0, atol=1e-12)
+
+    def reference_log_pdf():
+        import optuna
+        from optuna.samplers._tpe.parzen_estimator import _ParzenEstimator, _ParzenEstimatorParameters
+        from optuna.samplers._tpe.sampler import default_weights
+        names = [f"x{j:02d}" for j in range(P)]
+        space = {n: optuna.distributions.FloatDistribution(0.0, 1.0) for n in names}
+        prm = _ParzenEstimatorParameters(prior_weight=1.0, consider_magic_clip=True, consider_endpoints=False,
+                                         weights=default_weights, multivariate=True, categorical_distance_func={})
+        pts = {n: x[:, j] for j, n in enumerate(names)}
+        return [_ParzenEstimator({n: X[rows, j] for j, n in enumerate(names)}, space, prm).log_pdf(pts).tolist()
+                for rows in (above, below)]
+
+    logg, logl = recorded("test_fixture_points_against_oracle_and_live_reference/log_pdf", reference_log_pdf)
+    np.testing.assert_allclose(logg, g["logg"][pick], rtol=0, atol=1e-12)
+    np.testing.assert_allclose(logl, g["logl"][pick], rtol=0, atol=1e-12)

@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from optuna_b200 import _lib
+from tests._reference_golden import recorded
 from tests._util import draw_uniforms
 
 
@@ -42,13 +43,24 @@ def test_single_random_sample_call_is_the_reference_stream():
 
 
 def test_gamma_and_weights_mirror_reference_formulas():
-    optuna = pytest.importorskip("optuna")
-    from optuna.samplers._tpe import sampler as ref
+    pytest.importorskip("optuna")
     from optuna_b200.sampler import default_gamma, default_weights, hyperopt_default_gamma
-    for n in (0, 1, 10, 11, 24, 25, 26, 250, 100000):
-        assert default_gamma(n) == ref.default_gamma(n)
-        assert hyperopt_default_gamma(n) == ref.hyperopt_default_gamma(n)
-        assert np.array_equal(default_weights(n), ref.default_weights(n))
+    ns = (0, 1, 10, 11, 24, 25, 26, 250, 100000)
+
+    def sample(w):  # every weight of the short arrays, a fixed sample of the long one
+        idx = np.unique(np.r_[0:300, 300:len(w):997, len(w) - 300:len(w)])
+        return w[idx[(idx >= 0) & (idx < len(w))]]
+
+    def reference():
+        from optuna.samplers._tpe import sampler as ref
+        return [[ref.default_gamma(n), ref.hyperopt_default_gamma(n), sample(ref.default_weights(n)).tolist()]
+                for n in ns]
+
+    for n, (gamma, hyperopt_gamma, weights) in zip(ns, recorded("test_gamma_and_weights_mirror_reference_formulas",
+                                                                reference)):
+        assert default_gamma(n) == gamma
+        assert hyperopt_default_gamma(n) == hyperopt_gamma
+        assert np.array_equal(sample(default_weights(n)), np.asarray(weights, dtype=float))
 
 
 def test_sampler_constructor_contract():
@@ -73,12 +85,16 @@ def test_sampler_constructor_contract():
     with pytest.warns(FutureWarning):
         B200TPESampler(consider_prior=False)
     # startup trials never touch the device: they are optuna's RandomSampler (sampler.py:348-349, :471-474)
-    a = optuna.create_study(sampler=B200TPESampler(seed=0, n_startup_trials=5))
-    b = optuna.create_study(sampler=optuna.samplers.TPESampler(seed=0, n_startup_trials=5))
-    for s in (a, b):
+    def startup(sampler):
+        s = optuna.create_study(sampler=sampler)
         s.optimize(lambda t: t.suggest_float("x", 0, 1) + t.suggest_int("k", 1, 3)
                    + (t.suggest_categorical("c", ["u", None]) is None), n_trials=5)
-    assert [t.params for t in a.trials] == [t.params for t in b.trials] and a.sampler._engine is None
+        return s
+
+    a = startup(B200TPESampler(seed=0, n_startup_trials=5))
+    want = recorded("test_sampler_constructor_contract/startup",
+                    lambda: [t.params for t in startup(optuna.samplers.TPESampler(seed=0, n_startup_trials=5)).trials])
+    assert [t.params for t in a.trials] == want and a.sampler._engine is None
 
 
 def test_device_synced_rng_flushes_on_access_and_pickle():

@@ -1,5 +1,6 @@
-"""B200TPESampler behind the reference's OWN ``Study`` (unmodified optuna, oracle/_ref), compared live with
-``optuna.samplers.TPESampler`` driven through the same calls with the same seed.
+"""B200TPESampler behind the reference's OWN ``Study`` (unmodified optuna, oracle/_ref), compared with what
+``optuna.samplers.TPESampler`` computed when driven through the same calls with the same seed (stored in
+tests/golden/reference_runs.json.xz, see tests/_reference_golden.py).
 
 Every scenario runs twice: with the CPU oracle answering the array-level calls (checks the host glue -- trial
 log, device mirror, search spaces, RNG hand-over -- anywhere) and, marked ``gpu``, with libtpe_b200.so (the
@@ -16,6 +17,7 @@ optuna = pytest.importorskip("optuna")
 from optuna.samplers import TPESampler  # noqa: E402
 from optuna.trial import TrialState  # noqa: E402
 
+from tests._reference_golden import recorded, regenerating  # noqa: E402
 from tests._util import load  # noqa: E402
 
 warnings.filterwarnings("ignore", category=optuna.exceptions.ExperimentalWarning)
@@ -84,12 +86,16 @@ def over_seeds(scenario, make_sampler, ties, kw, seeds=(0, 1, 2, 3, 4, 5)):
     through without an acquisition tie; a difference that is not such a tie fails at once.  With the CPU oracle
     as the engine no tie is tolerated: glue + oracle must BE the reference."""
     base = kw.pop("seed", 0)
+    run = next(make_sampler.runs)
+    if regenerating():  # store the reference's run of every seed: the CUDA engine may need a later one
+        for seed in seeds:
+            make_sampler.yardstick(f"{run}/{base + seed}", scenario, ties, seed=base + seed, **kw)
     tied = []
     for seed in seeds:
         mine = make_sampler(seed=base + seed, **kw)
         audit = Audit(mine) if make_sampler.kind == "cuda" else None
         a = scenario(mine)
-        b = scenario(make_sampler.reference(ties, seed=base + seed, **kw))
+        b = make_sampler.yardstick(f"{run}/{base + seed}", scenario, ties, seed=base + seed, **kw)
         try:
             same_trials(a, b, audit)
             return a, b
@@ -138,8 +144,8 @@ def mixed(t):
 
 @pytest.mark.parametrize("mv", [False, True])
 def test_branin_200_trials_is_the_reference_trajectory(make_sampler, mv):
-    """BASELINE config 1: same seed => same 200-trial trajectory as optuna.samplers.TPESampler -- the live one
-    and the committed golden (tests/golden/branin.npz, generated from the reference by oracle/gen_golden.py)."""
+    """BASELINE config 1: same seed => same 200-trial trajectory as optuna.samplers.TPESampler (the committed
+    golden tests/golden/branin.npz, generated from the reference by oracle/gen_golden.py)."""
     study = optuna.create_study(sampler=make_sampler(seed=0, multivariate=mv))
     study.optimize(branin, n_trials=200)
     g = load("branin.npz")
@@ -151,10 +157,6 @@ def test_branin_200_trials_is_the_reference_trajectory(make_sampler, mv):
     assert study.sampler.ahead_stats[0] >= 180, study.sampler.ahead_stats
     if not mv:
         assert abs(study.best_value - 0.4069652013131506) < 1e-9
-    live = optuna.create_study(sampler=TPESampler(seed=0, multivariate=mv))
-    live.optimize(branin, n_trials=60)
-    for ta, tb in zip(study.trials, live.trials):
-        same(ta.params, tb.params)
 
 
 @pytest.mark.parametrize("mv", [False, True])
@@ -244,7 +246,7 @@ def test_group_decomposed_conditional_space(make_sampler):
     a, b = run_both(make_sampler, obj, 50, seed=4, multivariate=True, group=True, n_startup_trials=6)
     names = sorted(sorted(g) for g in a.sampler._groups_now)
     assert names == [["kind", "x"], ["ya"], ["yb", "zb"]]
-    assert [sorted(g) for g in a.sampler._groups_now] == [sorted(g) for g in b.sampler._search_space_group.search_spaces]
+    assert [sorted(g) for g in a.sampler._groups_now] == b.groups
     from optuna_b200 import B200TPESampler
     with pytest.raises(ValueError):
         B200TPESampler(group=True)
@@ -708,12 +710,16 @@ def test_batched_ask_equals_sequential_asks(make_sampler):
         s.optimize(obj, n_trials=30)
         return s
 
+    def params(trials):
+        return [[t.suggest_float(f"x{j}", 0, 1) for j in range(5)] + [t.suggest_int("k", 0, 9)] for t in trials]
+
+    def sequential():
+        b = warm(make_sampler.reference(**kw))
+        return params([b.ask() for _ in range(50)])
+
     kw = dict(seed=7, multivariate=True, n_ei_candidates=32)
-    a, b = warm(make_sampler(**kw)), warm(make_sampler.reference(**kw))
-    batch = ask_batch(a, 50)
-    seq = [b.ask() for _ in range(50)]
-    pa = [[t.suggest_float(f"x{j}", 0, 1) for j in range(5)] + [t.suggest_int("k", 0, 9)] for t in batch]
-    pb = [[t.suggest_float(f"x{j}", 0, 1) for j in range(5)] + [t.suggest_int("k", 0, 9)] for t in seq]
+    pa = params(ask_batch(warm(make_sampler(**kw)), 50))
+    pb = recorded("test_batched_ask_equals_sequential_asks/sequential", sequential)
     np.testing.assert_allclose(pa, pb, rtol=1e-9, atol=0)
     assert len({tuple(p) for p in pa}) > 40  # different uniforms per ask
 
@@ -745,8 +751,13 @@ def test_device_generated_uniforms_give_the_reference_suggestions(make_sampler):
                 sampler.close()                    # engine re-created at the next ask
         return got, sampler._rng.rng.random_sample(4)
 
+    def run_reference():
+        want, tail = run(make_sampler.reference(**kw))
+        return want, tail.tolist()
+
     kw = dict(seed=11, n_ei_candidates=C, multivariate=True)
-    (got, tail), (want, tail_ref) = run(make_sampler(**kw)), run(make_sampler.reference(**kw))
+    got, tail = run(make_sampler(**kw))
+    want, tail_ref = recorded("test_device_generated_uniforms_give_the_reference_suggestions/run", run_reference)
     np.testing.assert_allclose(got, want, rtol=1e-9, atol=0)
     assert np.array_equal(tail, tail_ref)  # the generator ends in the reference's state
 
