@@ -16,6 +16,7 @@ import json
 import math
 import threading
 import time
+from dataclasses import dataclass, field
 from typing import Any, Callable, Sequence
 
 import numpy as np
@@ -262,12 +263,17 @@ class _DeviceSyncedRng:
     Large asks draw their uniforms on the GPU; instead of copying the generator state back into the host
     ``RandomState`` after every ask (get_state + set_state cost 80 us), the state stays on the device
     and the next ask continues from it.  Any access to ``.rng`` -- an ask drawn on the host, reseeding,
-    pickling, somebody reading ``sampler._rng.rng`` -- first brings the host generator up to date."""
+    pickling, somebody reading ``sampler._rng.rng`` -- first brings the host generator up to date.
+
+    Work queued ahead of its ask `stage`s its draws without taking them: an undo armed with `arm` puts the generator
+    back to the snapshot taken before them (or, for a plan served in part, where the calls served so far left it).
+    Every staged draw is either adopted (`release(.., adopted=True)`) or undone -- by `release`, or by the next look
+    at ``.rng``, whichever comes first."""
 
     def __init__(self, inner) -> None:
         self._inner = inner
-        self._engine = None  # the engine holding a newer state, if any
-        self._settle = None  # a batch of per-parameter draws served only in part: call before anyone looks
+        self._engine = None  # the engine holding a newer state, if any (never while an undo is pending)
+        self._settle = None  # the pending undo: called before anyone looks
 
     @property
     def rng(self) -> np.random.RandomState:
@@ -284,6 +290,59 @@ class _DeviceSyncedRng:
 
     def mark_device(self, eng) -> None:
         self._engine = eng
+
+    def draw(self, eng, count: int, device: bool) -> np.ndarray | None:
+        """The next `count` uniforms for `eng`, taken at once: generated on the device (returns None), continuing
+        from the state `eng` holds if it holds one, or drawn on the host."""
+        if not device:
+            return self.rng.random_sample(count)
+        eng.stage_rng(None if self._engine is eng else self.rng, count)
+        self._engine = eng                            # from here on the device holds the newer state
+        return None
+
+    def stage(self, eng, count: int, device: bool) -> tuple[Any, np.ndarray | None]:
+        """Snapshot the generator and stage its next `count` uniforms for `eng` without taking them: generated on the
+        device, continuing from the state `eng` holds if it holds one, or drawn on the host (returned, else None).
+        Returns (snapshot, host draws).  Until the draws are adopted the generator stands at the snapshot: a caller
+        whose work fails `restore`s it, one whose work is queued `arm`s the undo."""
+        if not device:
+            r = self.rng                              # (a pending undo runs first)
+            snap = r.get_state()
+            return snap, r.random_sample(count)
+        if self._engine is eng:
+            snap = eng.rng_snapshot()                 # where the last ask left the generator (no device access)
+            eng.stage_rng(None, count)
+            self._engine = None
+        else:
+            r = self.rng
+            snap = r.get_state()
+            eng.stage_rng(r, count, state=snap)       # (the host object stays at the snapshot)
+        return snap, None
+
+    def restore(self, snap, advance: int = 0) -> None:
+        """Put the generator at `snap`, `advance` draws on."""
+        r = self._inner.rng
+        r.set_state(snap)
+        if advance:
+            r.random_sample(advance)
+        self._engine = None
+
+    def arm(self, undo: Callable[[], None]) -> Callable[[], None]:
+        """Make `undo` the pending undo of the draws just staged; returns it."""
+        self._settle = undo
+        return undo
+
+    def armed(self, undo) -> bool:
+        """Is `undo` still pending (nobody has looked at the generator since it was armed)?"""
+        return self._settle is undo
+
+    def release(self, undo, adopted: bool) -> None:
+        """The draws `undo` belongs to are adopted (the generator stays where they left it) or undone.  Nothing
+        happens when `undo` is no longer pending."""
+        if self._settle is undo:
+            self._settle = None
+            if not adopted:
+                undo()
 
     def __getstate__(self) -> dict:
         self.rng  # flush
@@ -308,6 +367,7 @@ class _Told:
         self.intermediate_values = dict(trial.intermediate_values)
         self.system_attrs = dict(trial.system_attrs)
         self.confirmed = False
+        self.threshold = None   # an outcome speculated by `_speculate`: the sort key the trial's value must not beat
 
     def matches(self, t) -> bool:
         """Is the stored trial exactly what was uploaded for it?"""
@@ -316,14 +376,25 @@ class _Told:
                 and t.system_attrs.get(CONSTRAINTS_KEY) == self.system_attrs.get(CONSTRAINTS_KEY))
 
 
+@dataclass(eq=False)
 class _Ahead:
-    """A suggestion whose device work was queued at ``tell`` time (``B200TPESampler._look_ahead``)."""
+    """A suggestion whose device work was queued before its ask (``B200TPESampler._look_ahead``, ``_speculate``)."""
 
-    def __init__(self, told, space, cols, cfg, dev_version, eng, dev_rng, cancel, kind="joint", **extra) -> None:
-        self.told, self.space, self.cols, self.cfg = told, space, cols, cfg
-        self.dev_version, self.eng, self.dev_rng, self.cancel = dev_version, eng, dev_rng, cancel
-        self.kind = kind                 # "joint": one sample_relative; "uni": the per-parameter calls of a trial
-        self.__dict__.update(extra)      # uni: order, wb, wa, snap
+    kind: str              # "joint": one sample_relative; "spec": the same, queued before the running trial ended;
+                           # "uni": the per-parameter calls of a trial
+    told: _Told            # the trial whose row was uploaded for it
+    space: dict
+    cols: list
+    cfg: dict
+    cfg_n_finished: int    # the count of finished trials `cfg` was made for ("spec" checks it at `tell` time)
+    dev_version: int
+    eng: Any
+    dev_rng: bool          # its uniforms were generated on the device
+    snap: Any              # the generator before its draws
+    cancel: Callable       # the undo armed on the generator for them
+    order: list = field(default_factory=list)  # "uni": the predicted calls, the user's weights of the two sets
+    wb: Any = None
+    wa: Any = None
 
 
 class _UniPlan:
@@ -345,6 +416,7 @@ class _UniPlan:
         self.prev: list = []       # calls of the last completed recording
         self.disabled = False      # the engine said "not batchable" for this space
         self.on_device = None      # the engine whose generator state is the one after the whole batch
+        self.settle = None         # the undo armed on the generator until the whole batch is served
 
 
 class B200TPESampler(BaseSampler):
@@ -610,20 +682,12 @@ class B200TPESampler(BaseSampler):
             if self._hist.n_finished < self._n_startup_trials:
                 return [{} for _ in range(n_asks)]
             cols = self._sync(study, None, search_space)
-            cfg = dict(n_below=int(self._gamma(self._hist.n_finished)), n_candidates=self._n_ei_candidates,
-                       multivariate=self._multivariate, prior_weight=self._prior_weight,
-                       magic_clip=self._magic_clip, endpoints=self._endpoints)
+            cfg = self._cfg(self._hist.n_finished)
             eng = self._eng()
-            multi = study._is_multi_objective()
-            _, nb, na = eng.prepare(cols, **cfg)
-            if self._weights is default_weights:
-                build = eng.build
-            else:
-                wb = None if multi else _checked_weights(self._weights, nb)
-                wa = _checked_weights(self._weights, na)
-                build = lambda: eng.build(wb, wa)  # noqa: E731
+            wb, wa = self._prepare(eng, cols, cfg, study)
+            eng.build(wb, wa)
             # ask-by-ask draws are consecutive stretches of one stream: one generation yields the same numbers
-            x = self._sample_and_select(eng, search_space, n_asks, build)
+            x = self._sample_and_select(eng, search_space, n_asks)
         # column-wise conversion (FloatDistribution.to_external_repr is the identity): 8192 x 32 values in
         # a few ms instead of one Python call per value
         names = list(search_space)
@@ -804,28 +868,46 @@ class B200TPESampler(BaseSampler):
         ONE call yields the identical stream (checked in tests/test_host_glue.py) at half the cost."""
         return self._rng.rng.random_sample(self._n_ei_candidates * (1 + len(search_space)))
 
-    def _sample_and_select(self, eng: TPEEngine, search_space: dict[str, BaseDistribution], n_asks: int,
-                           build) -> np.ndarray:
-        """Uniforms + stages 3-4.  Large asks: the library generates the generator's next outputs on the
-        GPU (k_mt19937_uniform, the same MT19937 stream bit for bit) while the estimator builds run, and the
-        host generator is moved to the state after the draws on demand; small asks draw on the host.  The
-        estimators are built (and validated) BEFORE the generator moves, as in the reference (sampler.py:544-553):
+    def _sample_and_select(self, eng: TPEEngine, search_space: dict[str, BaseDistribution], n_asks: int) -> np.ndarray:
+        """Uniforms + stages 3-4, once the estimators are built.  Large asks: the library generates the generator's
+        next outputs on the GPU (k_mt19937_uniform, the same MT19937 stream bit for bit) while the estimator builds
+        run, and the host generator is moved to the state after the draws on demand; small asks draw on the host.
+        The estimators are built (and validated) BEFORE the generator moves, as in the reference (sampler.py:544-553):
         an ask that fails in the build leaves the stream untouched."""
         n = n_asks * self._n_ei_candidates * (1 + len(search_space))
-        build()
-        if n >= self.DEVICE_RNG_MIN:
-            if self._rng.on_device(eng):
-                eng.stage_rng(None, n)            # continue from the state the previous ask ended in
-            else:
-                eng.stage_rng(self._rng.rng, n)
-            self._rng.mark_device(eng)            # from here on the device holds the newer state
-            x, _, _ = eng.sample_and_select(None, n_asks)
-        else:
-            x, _, _ = eng.sample_and_select(self._rng.rng.random_sample(n), n_asks)
+        x, _, _ = eng.sample_and_select(self._rng.draw(eng, n, n >= self.DEVICE_RNG_MIN), n_asks)
         return x
+
+    def _cfg(self, n_finished: int) -> dict:
+        """The configuration of every engine call, for a history of `n_finished` finished trials."""
+        if self._prior_weight < 0:
+            raise ValueError("A non-negative value must be specified for prior_weight,"
+                             f" but got {self._prior_weight}.")
+        return dict(n_below=int(self._gamma(n_finished)), n_candidates=self._n_ei_candidates,
+                    multivariate=self._multivariate, prior_weight=self._prior_weight, magic_clip=self._magic_clip,
+                    endpoints=self._endpoints)
+
+    def _prepare(self, eng: TPEEngine, cols: list[int], cfg: dict, study=None) -> tuple:
+        """``eng.prepare(cols)``, then the user's weights of the below and above sets as ``eng.build`` takes them --
+        None for `default_weights`, which the library evaluates itself (k_weights).  In a multi-objective `study`
+        l(x) is weighted by hypervolume contributions (computed by the library) and the user's function only
+        shapes g(x) (sampler.py:570-584)."""
+        _, nb, na = eng.prepare(cols, **cfg)
+        if self._weights is default_weights:
+            return None, None
+        wb = None if study is not None and study._is_multi_objective() else _checked_weights(self._weights, nb)
+        return wb, _checked_weights(self._weights, na)
 
     #: per-parameter asks of a univariate trial are evaluated together from this many parameters on
     UNI_BATCH_MIN = 2
+
+    def _plannable(self, study, calls: list) -> bool:
+        """Can the per-parameter `calls` of a trial be evaluated together (_UniPlan)?  Only for univariate TPE: the
+        reference computes a multivariate sampler's independent parameters with multivariate bandwidths
+        (sampler.py:335-341, :491), which the batched entry does not take."""
+        return (not self._multivariate and not self._constant_liar and not self._uni.disabled
+                and not study._is_multi_objective() and len(calls) >= self.UNI_BATCH_MIN
+                and len({n for n, _ in calls}) == len(calls))
 
     def _sample_one(self, study, trial, name: str, dist: BaseDistribution) -> Any:
         """One `sample_independent` past the startup trials.  The caller holds the lock and has polled."""
@@ -847,30 +929,16 @@ class B200TPESampler(BaseSampler):
             self._drop_ahead()
         if u.trial == trial.number and u.next < len(u.order):
             if u.order[u.next] == (name, dist) and u.version == version and not self._finished_backlog():
-                value = u.values[u.next]
-                u.next += 1
-                if u.next == len(u.order):           # served completely: the generator is where the batch left it
-                    self._rng._settle = None
-                    if u.on_device is not None:
-                        self._rng.mark_device(u.on_device)
-                return value
+                return self._serve_plan()
             self._rng.rng                            # not as predicted: settle the generator, then one at a time
             u.trial = None
-        can_batch = (not u.disabled and not self._constant_liar and not study._is_multi_objective()
-                     and len(u.prev) >= self.UNI_BATCH_MIN and u.prev[0] == (name, dist) and len(u.calls) == 1
-                     and len({n for n, _ in u.prev}) == len(u.prev))
-        if can_batch:
+        if len(u.calls) == 1 and u.prev and u.prev[0] == (name, dist) and self._plannable(study, u.prev):
             try:
-                self._plan_trial(study, trial, version)
+                return self._plan_trial(study, trial, version)
             except RuntimeError as e:
                 if "not batchable" not in str(e):
                     raise
                 u.disabled, u.trial = True, None
-            else:
-                u.next = 1
-                if len(u.order) == 1:
-                    self._rng._settle = None
-                return u.values[0]
         return self._sample(study, trial, {name: dist})[name]
 
     def _finished_backlog(self) -> bool:
@@ -878,47 +946,40 @@ class B200TPESampler(BaseSampler):
         h = self._hist
         return any(r not in h.pending for r in h.backlog)
 
-    def _plan_trial(self, study, trial, version) -> None:
-        """Evaluate every parameter of `self._uni.prev` for `trial` in one device call."""
-        u = self._uni
-        order = list(u.prev)
-        space = dict(order)
-        cols = self._sync(study, trial, space)
-        n = self._hist.n_finished
-        cfg = dict(n_below=int(self._gamma(n)), n_candidates=self._n_ei_candidates, multivariate=False,
-                   prior_weight=self._prior_weight, magic_clip=self._magic_clip, endpoints=self._endpoints)
-        if self._prior_weight < 0:
-            raise ValueError("A non-negative value must be specified for prior_weight,"
-                             f" but got {self._prior_weight}.")
-        eng = self._eng()
+    def _uni_batch(self, eng: TPEEngine, cols: list[int], cfg: dict, run) -> tuple:
+        """The user's weights and the uniforms of the per-parameter calls of `cols`, handed to `run`
+        (``eng.suggest_univariate_batch`` or its async twin).  Returns (what `run` returned, wb, wa, the generator
+        before the draws, whether they were generated on the device); if `run` fails, the generator is put back."""
         wb = wa = None
-        if self._weights is not default_weights:
-            _, nb, na = eng.prepare(cols[:1], **cfg)   # sizes of the two sets (the split does not depend on the column)
-            wb, wa = _checked_weights(self._weights, nb), _checked_weights(self._weights, na)
-        per = 2 * self._n_ei_candidates
-        count = per * len(order)
-        rng = self._rng.rng                            # host generator, up to date
-        st0 = rng.get_state()
+        if self._weights is not default_weights:   # the sizes of the two sets (the split does not depend on the column)
+            wb, wa = self._prepare(eng, cols[:1], cfg)
+        count = 2 * self._n_ei_candidates * len(cols)
+        dev_rng = count >= self.DEVICE_RNG_MIN
+        snap, uniforms = self._rng.stage(eng, count, dev_rng)
         try:
-            if count >= self.DEVICE_RNG_MIN:
-                eng.stage_rng(rng, count)              # the host object stays at st0 until the plan is served
-                x, _, _ = eng.suggest_univariate_batch(cols, None, wb, wa, **cfg)
-                u.on_device = eng
-            else:
-                x, _, _ = eng.suggest_univariate_batch(cols, rng.random_sample(count), wb, wa, **cfg)
-                u.on_device = None
+            out = run(cols, uniforms, wb, wa, **cfg)
         except Exception:
-            rng.set_state(st0)                         # nothing was served: the generator has not moved
+            self._rng.restore(snap)                 # nothing was served: the generator has not moved
             raise
-        self._install_plan(trial, version, order, cols, cfg, wb, wa, x, st0)
+        return out, wb, wa, snap, dev_rng
 
-    def _install_plan(self, trial, version, order, cols, cfg, wb, wa, x, st0) -> None:
-        """The batch has been evaluated (x: the winners per column, st0: the generator before its draws)."""
+    def _plan_trial(self, study, trial, version) -> Any:
+        """Evaluate every parameter of `self._uni.prev` for `trial` in one device call; returns the first value."""
+        order = list(self._uni.prev)
+        cols = self._sync(study, trial, dict(order))
+        cfg = self._cfg(self._hist.n_finished)
+        eng = self._eng()
+        (x, _, _), wb, wa, st0, dev_rng = self._uni_batch(eng, cols, cfg, eng.suggest_univariate_batch)
+        return self._install_plan(trial, version, order, cols, cfg, wb, wa, x, st0, eng if dev_rng else None)
+
+    def _install_plan(self, trial, version, order, cols, cfg, wb, wa, x, st0, on_device) -> Any:
+        """The batch has been evaluated (x: the winners per column, st0: the generator before its draws, on_device:
+        the engine that generated them, None for host draws); returns the first value."""
         u = self._uni
         eng = self._eng()
         per = 2 * self._n_ei_candidates
         count = per * len(order)
-        u.trial, u.order, u.version = trial.number, order, version
+        u.trial, u.order, u.version, u.on_device = trial.number, order, version, on_device
         u.values = [d.to_external_repr(float(v)) for (_, d), v in zip(order, x)]
         u.next = 0
         if self._audit is not None:
@@ -933,13 +994,21 @@ class B200TPESampler(BaseSampler):
                 self._audit(trial, {nm: d}, eng)
 
         def settle() -> None:   # the generator after the calls served so far (and only those)
-            r = self._rng._inner.rng
-            r.set_state(st0)
-            if u.next:
-                r.random_sample(per * u.next)
-            self._rng._engine = None
+            self._rng.restore(st0, per * u.next)
             u.trial = None
-        self._rng._settle = settle
+        u.settle = self._rng.arm(settle)
+        return self._serve_plan()
+
+    def _serve_plan(self) -> Any:
+        """The next value of the plan; once all are served the generator stands where the batch left it."""
+        u = self._uni
+        value = u.values[u.next]
+        u.next += 1
+        if u.next == len(u.order):
+            self._rng.release(u.settle, adopted=True)
+            if u.on_device is not None:
+                self._rng.mark_device(u.on_device)
+        return value
 
     def _look_ahead_uni(self, study, trial, state, values) -> None:
         """`_look_ahead` for univariate TPE: the per-parameter calls of the NEXT trial, predicted to repeat this
@@ -948,94 +1017,39 @@ class B200TPESampler(BaseSampler):
         the generator (`_adopt_uni_ahead`)."""
         self._drop_ahead()
         u = self._uni
-        if not (not self._constant_liar and not u.disabled and self._prior_weight >= 0
-                and (state == TrialState.COMPLETE or state == TrialState.PRUNED) and not study._is_multi_objective()
-                and u.calls_trial == trial.number and len(u.calls) >= self.UNI_BATCH_MIN
-                and len({n for n, _ in u.calls}) == len(u.calls)):
+        if not (self._prior_weight >= 0 and (state == TrialState.COMPLETE or state == TrialState.PRUNED)
+                and u.calls_trial == trial.number and self._plannable(study, u.calls)):
             return
-        h = self._hist
         order = list(u.calls)
         space = dict(order)
-        self._note_changes(self._poll(study))
-        if h.n_finished + 1 < self._n_startup_trials:
+        up = self._upload_told(study, trial, state, values, space)
+        if up is None:
             return
-        rng = self._rng
-        if rng._settle is not None:
-            rng.rng                                  # a half-served plan: settle the generator first
-        row = trial.number
-        cols = self._sync(study, None, space)
-        if row >= h.rows or row not in h.pending or h.numbers[row] != trial.number:
-            return
+        cols, told = up
         eng = self._eng()
-        told = _Told(trial, state, values)
-        if self._constraints_func is not None:
-            told.system_attrs[CONSTRAINTS_KEY] = study._storage.get_trial_system_attrs(trial._trial_id).get(CONSTRAINTS_KEY)
-        self._upload(study, eng, {row: told}, None)
-        h.dev_pred[row] = told
-        cfg = dict(n_below=int(self._gamma(h.n_finished + 1)), n_candidates=self._n_ei_candidates, multivariate=False,
-                   prior_weight=self._prior_weight, magic_clip=self._magic_clip, endpoints=self._endpoints)
-        per = 2 * self._n_ei_candidates
-        count = per * len(order)
-        inner = rng._inner
-        snap = None
-        wb = wa = None
+        cfg = self._cfg(self._hist.n_finished + 1)
         try:
-            if self._weights is not default_weights:
-                _, nb, na = eng.prepare(cols[:1], **cfg)
-                wb, wa = _checked_weights(self._weights, nb), _checked_weights(self._weights, na)
-            if count >= self.DEVICE_RNG_MIN:
-                if rng.on_device(eng):
-                    snap = eng.rng_snapshot()
-                    eng.stage_rng(None, count)
-                else:
-                    r = rng.rng
-                    snap = r.get_state()
-                    eng.stage_rng(r, count, state=snap)
-                eng.suggest_univariate_batch_async(cols, None, wb, wa, **cfg)
-                on_device = eng
-            else:
-                r = rng.rng
-                snap = r.get_state()
-                eng.suggest_univariate_batch_async(cols, r.random_sample(count), wb, wa, **cfg)
-                on_device = None
+            _, wb, wa, snap, dev_rng = self._uni_batch(eng, cols, cfg, eng.suggest_univariate_batch_async)
         except Exception:                            # e.g. "not batchable asynchronously": the ask plans as before
-            if snap is not None:
-                inner.rng.set_state(snap)
-                rng._engine = None
             return
-
-        def cancel() -> None:
-            inner.rng.set_state(snap)
-            rng._engine = None
-        rng._settle = cancel
-        self._ahead = _Ahead(told, space, cols, cfg, h.dev_version, eng, on_device is not None, cancel, kind="uni",
-                             order=order, wb=wb, wa=wa, snap=snap, on_device=on_device)
+        cancel = self._rng.arm(lambda: self._rng.restore(snap))
+        self._ahead = _Ahead("uni", told, space, cols, cfg, self._hist.n_finished + 1, self._hist.dev_version, eng,
+                             dev_rng, snap, cancel, order=order, wb=wb, wa=wa)
 
     def _adopt_uni_ahead(self, study, trial, a, name, dist, version) -> bool:
         """First `sample_independent` of a trial with a batch queued at `tell` time: take it if it is this trial's."""
-        self._ahead = None
         h = self._hist
         cols = self._sync(study, trial, dict(a.order))
-        cfg = dict(n_below=int(self._gamma(h.n_finished)), n_candidates=self._n_ei_candidates, multivariate=False,
-                   prior_weight=self._prior_weight, magic_clip=self._magic_clip, endpoints=self._endpoints)
-        ok = (a.told.confirmed and a.eng is self._engine and a.dev_version == h.dev_version and a.cols == cols
-              and a.cfg == cfg and a.order[0] == (name, dist) and self._rng._settle is a.cancel)
-        if not ok:
-            self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
+        cfg = self._cfg(h.n_finished)
+        if not (a.told.confirmed and a.eng is self._engine and a.dev_version == h.dev_version and a.cols == cols
+                and a.cfg == cfg and a.order[0] == (name, dist) and self._rng.armed(a.cancel)):
+            self._drop_ahead()
             return False
-        self._rng._settle = None
+        self._ahead = None
+        self._rng.release(a.cancel, adopted=True)
         x, _, _ = a.eng.collect_univariate()
-        u = self._uni
-        u.on_device = a.on_device                     # (host draws: the generator already stands after the batch)
-        self._install_plan(trial, version, a.order, cols, cfg, a.wb, a.wa, x, a.snap)
-        u.next = 1
-        if len(u.order) == 1:
-            self._rng._settle = None
-            if u.on_device is not None:
-                self._rng.mark_device(u.on_device)
+        # (host draws: the generator already stands after the batch)
+        self._install_plan(trial, version, a.order, cols, cfg, a.wb, a.wa, x, a.snap, a.eng if a.dev_rng else None)
         self.ahead_stats[0] += 1
         return True
 
@@ -1062,30 +1076,14 @@ class B200TPESampler(BaseSampler):
             # (prepare, build, uniforms, sampling + grids + argmax, read-back, to_external_repr)
             self.last_ask_s = (t1 - t0, time.perf_counter() - t1)
 
-    def _cfg(self, n_finished: int) -> dict:
-        return dict(n_below=int(self._gamma(n_finished)), n_candidates=self._n_ei_candidates,
-                    multivariate=self._multivariate, prior_weight=self._prior_weight, magic_clip=self._magic_clip,
-                    endpoints=self._endpoints)
-
     def _sample_synced(self, study, cols: list[int], search_space: dict[str, BaseDistribution]) -> dict[str, Any]:
         cfg = self._cfg(self._hist.n_finished)
-        if self._prior_weight < 0:
-            raise ValueError("A non-negative value must be specified for prior_weight,"
-                             f" but got {self._prior_weight}.")
         eng = self._eng()
         x = self._take_ahead(eng, cols, search_space, cfg)
-        if x is not None:
-            pass
-        elif self._weights is default_weights:
-            eng.prepare(cols, **cfg)
-            x = self._sample_and_select(eng, search_space, 1, eng.build)
-        else:
-            _, nb, na = eng.prepare(cols, **cfg)
-            # multi-objective studies weight l(x) by hypervolume contributions (computed by the
-            # library); the user's weights function then only shapes g(x) (sampler.py:570-584)
-            wb = None if study._is_multi_objective() else _checked_weights(self._weights, nb)
-            wa = _checked_weights(self._weights, na)
-            x = self._sample_and_select(eng, search_space, 1, lambda: eng.build(wb, wa))
+        if x is None:
+            wb, wa = self._prepare(eng, cols, cfg, study)
+            eng.build(wb, wa)
+            x = self._sample_and_select(eng, search_space, 1)
         self._last_space = search_space
         out = {}
         for j, (name, d) in enumerate(search_space.items()):
@@ -1101,43 +1099,57 @@ class B200TPESampler(BaseSampler):
         rebuild the device history from the study (nothing the device holds is trusted)."""
         try:
             self._drop_ahead()
-        except Exception:
-            self._ahead = None
-            self._rng._settle = None
+        except Exception:                            # (the failed undo is no longer pending)
+            pass
         h = self._hist
         h.dev_token = None
         h.dev_pred.clear()
 
     def _drop_ahead(self) -> None:
+        """Discard the suggestion queued ahead, if any: nobody takes it, its draws are undone."""
         a, self._ahead = self._ahead, None
         if a is not None:
             self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
+            self._rng.release(a.cancel, adopted=False)
 
     def _take_ahead(self, eng, cols, search_space, cfg):
         """The suggestion queued at `tell` time, if this ask is the one it was computed for: the very columns and
         configuration, the finished trial stored exactly as it was uploaded, nothing else the estimators see
         changed since, the generator untouched.  Otherwise the generator goes back to where it was."""
-        a, self._ahead = self._ahead, None
+        a = self._ahead
         if a is None:
             return None
-        ok = (a.kind == "joint" and a.told.confirmed and a.eng is eng and a.dev_version == self._hist.dev_version and a.cols == cols
-              and a.cfg == cfg and self._rng._settle is a.cancel
-              and list(a.space.items()) == list(search_space.items()))
-        if not ok:
-            self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
+        if not (a.kind == "joint" and a.told.confirmed and a.eng is eng and a.dev_version == self._hist.dev_version
+                and a.cols == cols and a.cfg == cfg and self._rng.armed(a.cancel)
+                and list(a.space.items()) == list(search_space.items())):
+            self._drop_ahead()
             return None
-        self._rng._settle = None
+        self._ahead = None
+        self._rng.release(a.cancel, adopted=True)
         x, _, _ = eng.collect()
         if a.dev_rng:
             self._rng.mark_device(eng)
         self.ahead_stats[0] += 1
         return x
+
+    def _upload_told(self, study, trial, state, values, space) -> tuple[list[int], _Told] | None:
+        """`tell` time, past the startup trials: the finished trial's row goes to the device before the storage
+        shows it.  Returns the device columns of `space` and what was uploaded, or None when the trial's row is not
+        the log's pending row of that trial (nothing is uploaded then)."""
+        h = self._hist
+        self._note_changes(self._poll(study))
+        if h.n_finished + 1 < self._n_startup_trials:
+            return None
+        row = trial.number
+        cols = self._sync(study, None, space)
+        if row >= h.rows or row not in h.pending or h.numbers[row] != trial.number:
+            return None
+        told = _Told(trial, state, values)
+        if self._constraints_func is not None:       # after_trial has just stored them (samplers/_base.py:241-267)
+            told.system_attrs[CONSTRAINTS_KEY] = study._storage.get_trial_system_attrs(trial._trial_id).get(CONSTRAINTS_KEY)
+        self._upload(study, self._eng(), {row: told}, None)
+        h.dev_pred[row] = told                       # (_upload kept its category in dev_cat: the row is pending)
+        return cols, told
 
     def _look_ahead(self, study, trial, state, values) -> None:
         """Called from `after_trial`: the trial, its final state and values are known, the storage records them
@@ -1153,25 +1165,14 @@ class B200TPESampler(BaseSampler):
         if not (self._multivariate and not self._group and not self._constant_liar and self._prior_weight >= 0
                 and (state == TrialState.COMPLETE or state == TrialState.PRUNED)):
             return
-        h = self._hist
         space = self._last_space
         d = trial.distributions
         if any(d.get(k) != v for k, v in space.items()):
             return                                   # the intersection search space shrinks with this trial
-        self._note_changes(self._poll(study))
-        if h.n_finished + 1 < self._n_startup_trials:
-            return
-        row = trial.number
-        cols = self._sync(study, None, space)
-        if row >= h.rows or row not in h.pending or h.numbers[row] != trial.number:
-            return
-        eng = self._eng()
-        told = _Told(trial, state, values)
-        if self._constraints_func is not None:       # after_trial has just stored them (samplers/_base.py:241-267)
-            told.system_attrs[CONSTRAINTS_KEY] = study._storage.get_trial_system_attrs(trial._trial_id).get(CONSTRAINTS_KEY)
-        self._upload(study, eng, {row: told}, None)
-        h.dev_pred[row] = told                       # (_upload kept its category in dev_cat: the row is pending)
-        self._queue_ahead(study, cols, space, told, "joint")
+        up = self._upload_told(study, trial, state, values, space)
+        if up is not None:
+            cols, told = up
+            self._queue_ahead(study, cols, space, told, "joint")
 
     def _confirm_speculation(self, study, trial, state, values) -> bool:
         """`tell` time: did the trial end the way `_speculate` assumed?  Then the queued suggestion is the next one's;
@@ -1182,7 +1183,7 @@ class B200TPESampler(BaseSampler):
         h = self._hist
         g = a.told
         ok = (g.number == trial.number and state == TrialState.COMPLETE and values is not None and len(values) == 1
-              and self._rng._settle is a.cancel and a.dev_version == h.dev_version and a.eng is self._engine
+              and self._rng.armed(a.cancel) and a.dev_version == h.dev_version and a.eng is self._engine
               and trial.params == g.params and trial.distributions == g.distributions)
         if ok:
             v = float(values[0])
@@ -1202,54 +1203,29 @@ class B200TPESampler(BaseSampler):
         self.spec_stats[0] += 1
         return True
 
-    def _queue_ahead(self, study, cols, space, told, kind) -> bool:
+    def _queue_ahead(self, study, cols, space, told, kind) -> None:
         """Queue the joint suggestion of the ask after `told` (whose row is on the device) without waiting for it."""
         h = self._hist
         eng = self._eng()
         cfg = self._cfg(h.n_finished + 1)
         n = self._n_ei_candidates * (1 + len(space))
-        rng = self._rng
-        if rng._settle is not None:
-            rng.rng                                  # a half-served batch of per-parameter draws: settle it first
-        inner = rng._inner
+        dev_rng = n >= self.DEVICE_RNG_MIN
         snap = None
         try:
-            dev_rng = n >= self.DEVICE_RNG_MIN
-            staged = None
             if not dev_rng:                          # host draws: uploaded on the side stream before anything is queued
-                r = rng.rng                          # (a copy from pageable memory waits for the work queued before it)
-                snap = r.get_state()
-                staged = eng.stage_uniforms(r.random_sample(n))
-            _, nb, na = eng.prepare(cols, **cfg)
-            if self._weights is default_weights:
-                eng.build()
-            else:                                    # as _sample_synced (sampler.py:570-584)
-                eng.build(None if study._is_multi_objective() else _checked_weights(self._weights, nb),
-                          _checked_weights(self._weights, na))
-            if dev_rng and rng.on_device(eng):
-                snap = eng.rng_snapshot()            # where the last ask left the generator (no device access)
-                eng.stage_rng(None, n)
-                eng.sample_and_select_async(None, 1)
-            elif dev_rng:
-                r = rng.rng
-                snap = r.get_state()
-                eng.stage_rng(r, n, state=snap)
-                eng.sample_and_select_async(None, 1)
-            else:
-                eng.sample_and_select_async(staged, 1)
+                snap, uniforms = self._rng.stage(eng, n, False)  # (a copy from pageable memory waits for the work
+                uniforms = eng.stage_uniforms(uniforms)          # queued before it)
+            wb, wa = self._prepare(eng, cols, cfg, study)        # as _sample_synced
+            eng.build(wb, wa)
+            if dev_rng:
+                snap, uniforms = self._rng.stage(eng, n, True)
+            eng.sample_and_select_async(uniforms, 1)
         except Exception:                            # the ask will run into it again, and report it
             if snap is not None:
-                inner.rng.set_state(snap)
-                rng._engine = None
-            return False
-
-        def cancel() -> None:                        # nobody took the suggestion: the draws never happened
-            inner.rng.set_state(snap)
-            rng._engine = None
-        rng._settle = cancel
-        self._ahead = _Ahead(told, space, cols, cfg, h.dev_version, eng, dev_rng, cancel, kind=kind,
-                             cfg_n_finished=h.n_finished + 1)
-        return True
+                self._rng.restore(snap)
+            return
+        cancel = self._rng.arm(lambda: self._rng.restore(snap))   # nobody took the suggestion: the draws never happened
+        self._ahead = _Ahead(kind, told, space, cols, cfg, h.n_finished + 1, h.dev_version, eng, dev_rng, snap, cancel)
 
     #: queue the NEXT suggestion already when a suggestion has been handed out, assuming the trial will end up in the
     #: above set (see _speculate)
@@ -1282,264 +1258,3 @@ class B200TPESampler(BaseSampler):
         self._upload(study, self._eng(), {row: guess}, None)
         h.dev_pred[row] = guess
         self._queue_ahead(study, cols, space, guess, "spec")
-
-    def _look_ahead_uni(self, study, trial, state, values) -> None:
-        """`_look_ahead` for univariate TPE: the per-parameter calls of the NEXT trial, predicted to repeat this
-        trial's, are queued as one batch now (tpe_suggest_univariate_batch_async); the first `sample_independent` of
-        the next trial adopts it if the trial was stored as uploaded, the call is the predicted one and nobody touched
-        the generator (`_adopt_uni_ahead`)."""
-        self._drop_ahead()
-        u = self._uni
-        if not (not self._constant_liar and not u.disabled and self._prior_weight >= 0
-                and (state == TrialState.COMPLETE or state == TrialState.PRUNED) and not study._is_multi_objective()
-                and u.calls_trial == trial.number and len(u.calls) >= self.UNI_BATCH_MIN
-                and len({n for n, _ in u.calls}) == len(u.calls)):
-            return
-        h = self._hist
-        order = list(u.calls)
-        space = dict(order)
-        self._note_changes(self._poll(study))
-        if h.n_finished + 1 < self._n_startup_trials:
-            return
-        rng = self._rng
-        if rng._settle is not None:
-            rng.rng                                  # a half-served plan: settle the generator first
-        row = trial.number
-        cols = self._sync(study, None, space)
-        if row >= h.rows or row not in h.pending or h.numbers[row] != trial.number:
-            return
-        eng = self._eng()
-        told = _Told(trial, state, values)
-        if self._constraints_func is not None:
-            told.system_attrs[CONSTRAINTS_KEY] = study._storage.get_trial_system_attrs(trial._trial_id).get(CONSTRAINTS_KEY)
-        self._upload(study, eng, {row: told}, None)
-        h.dev_pred[row] = told
-        cfg = dict(n_below=int(self._gamma(h.n_finished + 1)), n_candidates=self._n_ei_candidates, multivariate=False,
-                   prior_weight=self._prior_weight, magic_clip=self._magic_clip, endpoints=self._endpoints)
-        per = 2 * self._n_ei_candidates
-        count = per * len(order)
-        inner = rng._inner
-        snap = None
-        wb = wa = None
-        try:
-            if self._weights is not default_weights:
-                _, nb, na = eng.prepare(cols[:1], **cfg)
-                wb, wa = _checked_weights(self._weights, nb), _checked_weights(self._weights, na)
-            if count >= self.DEVICE_RNG_MIN:
-                if rng.on_device(eng):
-                    snap = eng.rng_snapshot()
-                    eng.stage_rng(None, count)
-                else:
-                    r = rng.rng
-                    snap = r.get_state()
-                    eng.stage_rng(r, count, state=snap)
-                eng.suggest_univariate_batch_async(cols, None, wb, wa, **cfg)
-                on_device = eng
-            else:
-                r = rng.rng
-                snap = r.get_state()
-                eng.suggest_univariate_batch_async(cols, r.random_sample(count), wb, wa, **cfg)
-                on_device = None
-        except Exception:                            # e.g. "not batchable asynchronously": the ask plans as before
-            if snap is not None:
-                inner.rng.set_state(snap)
-                rng._engine = None
-            return
-
-        def cancel() -> None:
-            inner.rng.set_state(snap)
-            rng._engine = None
-        rng._settle = cancel
-        self._ahead = _Ahead(told, space, cols, cfg, h.dev_version, eng, on_device is not None, cancel, kind="uni",
-                             order=order, wb=wb, wa=wa, snap=snap, on_device=on_device)
-
-    def _adopt_uni_ahead(self, study, trial, a, name, dist, version) -> bool:
-        """First `sample_independent` of a trial with a batch queued at `tell` time: take it if it is this trial's."""
-        self._ahead = None
-        h = self._hist
-        cols = self._sync(study, trial, dict(a.order))
-        cfg = dict(n_below=int(self._gamma(h.n_finished)), n_candidates=self._n_ei_candidates, multivariate=False,
-                   prior_weight=self._prior_weight, magic_clip=self._magic_clip, endpoints=self._endpoints)
-        ok = (a.told.confirmed and a.eng is self._engine and a.dev_version == h.dev_version and a.cols == cols
-              and a.cfg == cfg and a.order[0] == (name, dist) and self._rng._settle is a.cancel)
-        if not ok:
-            self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
-            return False
-        self._rng._settle = None
-        x, _, _ = a.eng.collect_univariate()
-        u = self._uni
-        u.on_device = a.on_device                     # (host draws: the generator already stands after the batch)
-        self._install_plan(trial, version, a.order, cols, cfg, a.wb, a.wa, x, a.snap)
-        u.next = 1
-        if len(u.order) == 1:
-            self._rng._settle = None
-            if u.on_device is not None:
-                self._rng.mark_device(u.on_device)
-        self.ahead_stats[0] += 1
-        return True
-
-    def _sample(self, study, trial, search_space: dict[str, BaseDistribution], speculate: bool = False) -> dict[str, Any]:
-        """TPESampler._sample (sampler.py:523-560).  The caller holds the lock and has polled."""
-        t0 = time.perf_counter()
-        cols = self._sync(study, trial, search_space)
-        t1 = time.perf_counter()
-        try:
-            out = self._sample_synced(study, cols, search_space)
-            if self._audit is not None:
-                self._audit(trial, search_space, self._eng())
-            if speculate and self.LOOK_AHEAD and self.SPECULATE:
-                t2 = time.perf_counter()
-                try:
-                    self._speculate(study, trial, cols, search_space, out)
-                except Exception as e:               # ... nor an `ask` whose suggestion is already computed
-                    _logger.debug(f"speculation abandoned: {e!r}")
-                    self._abandon_ahead()
-                self.last_spec_s = time.perf_counter() - t2
-            return out
-        finally:
-            # wall time of the last ask: history sync (host walk + row uploads) / everything after it
-            # (prepare, build, uniforms, sampling + grids + argmax, read-back, to_external_repr)
-            self.last_ask_s = (t1 - t0, time.perf_counter() - t1)
-
-    def _cfg(self, n_finished: int) -> dict:
-        return dict(n_below=int(self._gamma(n_finished)), n_candidates=self._n_ei_candidates,
-                    multivariate=self._multivariate, prior_weight=self._prior_weight, magic_clip=self._magic_clip,
-                    endpoints=self._endpoints)
-
-    def _sample_synced(self, study, cols: list[int], search_space: dict[str, BaseDistribution]) -> dict[str, Any]:
-        cfg = self._cfg(self._hist.n_finished)
-        if self._prior_weight < 0:
-            raise ValueError("A non-negative value must be specified for prior_weight,"
-                             f" but got {self._prior_weight}.")
-        eng = self._eng()
-        x = self._take_ahead(eng, cols, search_space, cfg)
-        if x is not None:
-            pass
-        elif self._weights is default_weights:
-            eng.prepare(cols, **cfg)
-            x = self._sample_and_select(eng, search_space, 1, eng.build)
-        else:
-            _, nb, na = eng.prepare(cols, **cfg)
-            # multi-objective studies weight l(x) by hypervolume contributions (computed by the
-            # library); the user's weights function then only shapes g(x) (sampler.py:570-584)
-            wb = None if study._is_multi_objective() else _checked_weights(self._weights, nb)
-            wa = _checked_weights(self._weights, na)
-            x = self._sample_and_select(eng, search_space, 1, lambda: eng.build(wb, wa))
-        self._last_space = search_space
-        out = {}
-        for j, (name, d) in enumerate(search_space.items()):
-            out[name] = d.to_external_repr(float(x[0, j]))
-        return out
-
-    # -- look-ahead: the next suggestion is computed while the study finishes `tell` and starts `ask` ----------
-    #: queue the next joint suggestion at `tell` time (multivariate TPE; see _look_ahead)
-    LOOK_AHEAD = True
-
-    def _drop_ahead(self) -> None:
-        a, self._ahead = self._ahead, None
-        if a is not None:
-            self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
-
-    def _take_ahead(self, eng, cols, search_space, cfg):
-        """The suggestion queued at `tell` time, if this ask is the one it was computed for: the very columns and
-        configuration, the finished trial stored exactly as it was uploaded, nothing else the estimators see
-        changed since, the generator untouched.  Otherwise the generator goes back to where it was."""
-        a, self._ahead = self._ahead, None
-        if a is None:
-            return None
-        ok = (a.kind == "joint" and a.told.confirmed and a.eng is eng and a.dev_version == self._hist.dev_version and a.cols == cols
-              and a.cfg == cfg and self._rng._settle is a.cancel
-              and list(a.space.items()) == list(search_space.items()))
-        if not ok:
-            self.ahead_stats[1] += 1
-            if self._rng._settle is a.cancel:
-                self._rng._settle = None
-                a.cancel()
-            return None
-        self._rng._settle = None
-        x, _, _ = eng.collect()
-        if a.dev_rng:
-            self._rng.mark_device(eng)
-        self.ahead_stats[0] += 1
-        return x
-
-    def _look_ahead(self, study, trial, state, values) -> None:
-        """Called from `after_trial`: the trial, its final state and values are known, the storage records them
-        right after (study/_tell.py:163-169).  In a sequential loop everything the next ask will compute is
-        determined at this point -- the history plus this trial, the same search space, the generator where the
-        last ask left it -- so the row is uploaded and the whole suggestion queued on the device now; it runs while
-        optuna stores the trial and creates the next one, and `sample_relative` collects it after checking that the
-        ask really is the predicted one (`_take_ahead`).  Joint sampling only; anything out of the ordinary (constant
-        liar, groups, a failed trial, a changed space) just skips it."""
-        if self._confirm_speculation(study, trial, state, values):
-            return
-        self._drop_ahead()
-        if not (self._multivariate and not self._group and not self._constant_liar and self._prior_weight >= 0
-                and (state == TrialState.COMPLETE or state == TrialState.PRUNED)):
-            return
-        h = self._hist
-        space = self._last_space
-        d = trial.distributions
-        if any(d.get(k) != v for k, v in space.items()):
-            return                                   # the intersection search space shrinks with this trial
-        self._note_changes(self._poll(study))
-        if h.n_finished + 1 < self._n_startup_trials:
-            return
-        row = trial.number
-        cols = self._sync(study, None, space)
-        if row >= h.rows or row not in h.pending or h.numbers[row] != trial.number:
-            return
-        eng = self._eng()
-        told = _Told(trial, state, values)
-        if self._constraints_func is not None:       # after_trial has just stored them (samplers/_base.py:241-267)
-            told.system_attrs[CONSTRAINTS_KEY] = study._storage.get_trial_system_attrs(trial._trial_id).get(CONSTRAINTS_KEY)
-        self._upload(study, eng, {row: told}, None)
-        h.dev_pred[row] = told                       # (_upload kept its category in dev_cat: the row is pending)
-        cfg = self._cfg(h.n_finished + 1)
-        n = self._n_ei_candidates * (1 + len(space))
-        rng = self._rng
-        if rng._settle is not None:
-            rng.rng                                  # a half-served batch of per-parameter draws: settle it first
-        inner = rng._inner
-        snap = None
-        try:
-            dev_rng = n >= self.DEVICE_RNG_MIN
-            staged = None
-            if not dev_rng:                          # host draws: uploaded on the side stream before anything is queued
-                r = rng.rng                          # (a copy from pageable memory waits for the work queued before it)
-                snap = r.get_state()
-                staged = eng.stage_uniforms(r.random_sample(n))
-            _, nb, na = eng.prepare(cols, **cfg)
-            if self._weights is default_weights:
-                eng.build()
-            else:                                    # as _sample_synced (sampler.py:570-584)
-                eng.build(None if study._is_multi_objective() else _checked_weights(self._weights, nb),
-                          _checked_weights(self._weights, na))
-            if dev_rng and rng.on_device(eng):
-                snap = eng.rng_snapshot()            # where the last ask left the generator (no device access)
-                eng.stage_rng(None, n)
-                eng.sample_and_select_async(None, 1)
-            elif dev_rng:
-                r = rng.rng
-                snap = r.get_state()
-                eng.stage_rng(r, n, state=snap)
-                eng.sample_and_select_async(None, 1)
-            else:
-                eng.sample_and_select_async(staged, 1)
-        except Exception:                            # the ask will run into it again, and report it
-            if snap is not None:
-                inner.rng.set_state(snap)
-                rng._engine = None
-            return
-
-        def cancel() -> None:                        # nobody took the suggestion: the draws never happened
-            inner.rng.set_state(snap)
-            rng._engine = None
-        rng._settle = cancel
-        self._ahead = _Ahead(told, space, cols, cfg, h.dev_version, eng, dev_rng, cancel)

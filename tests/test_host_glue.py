@@ -125,6 +125,24 @@ def test_device_synced_rng_flushes_on_access_and_pickle():
     assert np.array_equal(clone.rng.random_sample(4), want)
     assert np.array_equal(proxy.rng.random_sample(4), want) and eng.calls == 1
 
+    # draws staged ahead of their ask: an armed undo puts the generator back at the next look, a released one does not
+    before = proxy.rng.get_state()
+    snap, drawn = proxy.stage(eng, 6, device=False)
+    assert np.array_equal(drawn, ahead.random_sample(6))
+    undo = proxy.arm(lambda: proxy.restore(snap))
+    assert proxy.armed(undo)
+    assert np.array_equal(proxy.rng.random_sample(6), drawn) and not proxy.armed(undo)   # undone before the look
+    proxy.rng.set_state(before)
+    snap, drawn = proxy.stage(eng, 6, device=False)
+    undo = proxy.arm(lambda: proxy.restore(snap))
+    proxy.release(undo, adopted=True)
+    assert not proxy.armed(undo)
+    assert np.array_equal(proxy.rng.random_sample(4), ahead.random_sample(4))           # nothing restored
+    undo = proxy.arm(lambda: proxy.restore(snap, 2))           # a plan served in part: restored `advance` draws on
+    proxy.release(undo, adopted=False)
+    assert np.array_equal(proxy.rng.random_sample(4), drawn[2:])
+    assert not pickle.loads(pickle.dumps(proxy)).armed(undo) and eng.calls == 1
+
 
 def test_trial_log_matches_optunas_search_spaces_under_out_of_order_finishes():
     """_History.poll / intersection / group_spaces vs optuna's IntersectionSearchSpace

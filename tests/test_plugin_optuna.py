@@ -262,6 +262,16 @@ def test_conditional_space_without_group_warns_and_matches(make_sampler):
     run_both(make_sampler, obj, 40, seed=8, multivariate=True, n_startup_trials=6)
     run_both(make_sampler, obj, 40, ties=True, seed=8, multivariate=False, n_startup_trials=6)
 
+    # a multivariate sampler's independent parameters use multivariate bandwidths (sampler.py:335-341, :491), also
+    # when two or more of them are asked in the same order in every trial
+    def obj2(t):
+        hi = 4.0 if t.number == 0 else 3.0   # trial 0 keeps x and y out of the intersection search space
+        x = t.suggest_float("x", -3.0, hi)
+        y = t.suggest_float("y", -3.0, hi)
+        return (x - 1) ** 2 + (y + 0.5) ** 2
+
+    run_both(make_sampler, obj2, 30, seed=3, multivariate=True, n_startup_trials=5)
+
 
 def test_categorical_distance_func(make_sampler):
     def obj(t):
