@@ -35,7 +35,8 @@ extern "C" {
 /* 4: + tpe_sample_and_select_async / tpe_collect */
 /* 5: + tpe_suggest_univariate_batch_async / tpe_collect_univariate */
 /* 6: + tpe_set_kernel_shard / tpe_sample_and_partial / tpe_finish_from_partials */
-#define TPE_ABI_VERSION 6
+/* 7: + tpe_ped_anova */
+#define TPE_ABI_VERSION 7
 
 enum {
   TPE_OK = 0,
@@ -270,6 +271,37 @@ int tpe_last_timing(tpe_ctx* ctx, float* ms9, int32_t* launches);
 int tpe_probe_fp64_tflops(tpe_ctx* ctx, double* tflops);
 /* Which kernel variant the last log-density pass used (static string). */
 const char* tpe_last_logpdf_kernel(tpe_ctx* ctx);
+
+/* ---- PED-ANOVA hyperparameter importance ---------------------------------------------------------------------
+ * Replaces PedAnovaImportanceEvaluator.evaluate after its search-space walk (optuna/importance/_ped_anova/
+ * evaluator.py:222-266): _get_filtered_trials (importance/_base.py:145-156), _QuantileFilter.filter
+ * (evaluator.py:37-55), the binning of scott_parzen_estimator.py:90-135, _ScottParzenEstimator
+ * (scott_parzen_estimator.py:16-87) and _compute_pearson_divergence (evaluator.py:196-220), on the resident history.
+ * Fields are the evaluator's constructor arguments and its fixed settings (evaluator.py:141-172):
+ * prior_weight (> 0; 1.0), min_n_top (2) and n_steps (<= 128; 50). */
+typedef struct {
+  double target_quantile, region_quantile, prior_weight;
+  int32_t evaluate_on_local, min_n_top, n_steps;
+} tpe_ped_cfg;
+
+/* A row is kept when its category is TPE_CAT_COMPLETE, none of cols[] is NaN and its loss is finite.  The loss is
+ * key[r][0] (the sign-normalised objective) or loss[r] (a host-evaluated target; length = history size).  The target
+ * set is the kept rows with loss <= the k-th smallest kept loss, k = max(min_n_top - 1, ceil(q * n) - 1) at
+ * q = target_quantile; the region set likewise at region_quantile, or every kept row when it is 1.0.
+ *   cols       [n_cols] columns to filter on and evaluate
+ *   grids      [n_cols][n_steps] np.linspace grid of each numerical column (log domain for log columns), as the host
+ *              computes it (scott_parzen_estimator.py:96-105); ignored for categorical columns; may be NULL when
+ *              every column is categorical
+ *   n_grid     [n_cols] bins per column: <= n_steps, or n_choices for a categorical column
+ *   loss       [history size] or NULL = key[:, 0]
+ *   out_importance [n_cols] (n_target / n_region)^2 * Pearson divergence; all 0 when n_kept <= min_n_top
+ *   out_n      [3] kept, target, region (target = region = 0 when n_kept <= min_n_top)
+ *   out_counts optional [n_cols][2][max n_grid]: target / region histograms (inspection)
+ * Runs on the context stream, returns when the results are on the host, and leaves the history, the split and the
+ * estimators of the suggestion path untouched. */
+int tpe_ped_anova(tpe_ctx* ctx, const tpe_ped_cfg* cfg, const int32_t* cols, int32_t n_cols, const double* grids,
+                  const int32_t* n_grid, const double* loss, double* out_importance, int64_t* out_n,
+                  int32_t* out_counts);
 
 #ifdef __cplusplus
 }

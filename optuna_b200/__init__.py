@@ -6,11 +6,14 @@ sm_100a CUDA through a C ABI (include/optuna_b200_tpe.h) bound with ctypes.
 """
 from .engine import ParamSpec, TPEEngine  # noqa: F401
 
-__all__ = ["ParamSpec", "TPEEngine", "B200TPESampler"]
+__all__ = ["ParamSpec", "TPEEngine", "B200TPESampler", "B200PedAnovaImportanceEvaluator"]
 
 
 def __getattr__(name):
     if name == "B200TPESampler":
         from .sampler import B200TPESampler
         return B200TPESampler
+    if name == "B200PedAnovaImportanceEvaluator":
+        from .importance import B200PedAnovaImportanceEvaluator
+        return B200PedAnovaImportanceEvaluator
     raise AttributeError(name)

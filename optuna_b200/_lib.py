@@ -31,6 +31,11 @@ class SplitInfo(C.Structure):
     _fields_ = [("n_below_all", C.c_int64), ("n_below_obs", C.c_int64), ("n_above_obs", C.c_int64)]
 
 
+class PedCfg(C.Structure):
+    _fields_ = [("target_quantile", C.c_double), ("region_quantile", C.c_double), ("prior_weight", C.c_double),
+                ("evaluate_on_local", C.c_int32), ("min_n_top", C.c_int32), ("n_steps", C.c_int32)]
+
+
 # name -> (restype, argtypes); every symbol include/optuna_b200_tpe.h declares
 _P = C.c_void_p
 SYMBOLS = {
@@ -75,12 +80,13 @@ SYMBOLS = {
     "tpe_last_timing": (C.c_int, [_P, _P, _P]),
     "tpe_probe_fp64_tflops": (C.c_int, [_P, C.POINTER(C.c_double)]),
     "tpe_last_logpdf_kernel": (C.c_char_p, [_P]),
+    "tpe_ped_anova": (C.c_int, [_P, C.POINTER(PedCfg), _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None
 
 
-ABI_VERSION = 6  # include/optuna_b200_tpe.h TPE_ABI_VERSION
+ABI_VERSION = 7  # include/optuna_b200_tpe.h TPE_ABI_VERSION
 
 
 def load() -> C.CDLL:

@@ -23,6 +23,7 @@
 #include "tpe_mixed.cuh"
 #include "tpe_tcscreen.cuh"
 #include "tpe_unib.cuh"
+#include "tpe_importance.cuh"
 // Lab build (-DTPE_LAB): the experimental grid kernels and the timing-attribution variants measured in
 // profiles/r1_variants.md / r2_variants.md, selectable by environment variables.  Some of them switch parts of the
 // log-sum-exp off (wrong results by design).  The product library contains none of them.
@@ -244,6 +245,8 @@ struct tpe_ctx {
   uint64_t uni_ord_lineage = 0;        // ... and what else it belongs to
   int32_t uni_ord_col = -1;
   int64_t uni_ord_K = -1;
+  // PED-ANOVA importance (tpe_ped_anova): scratch of its own, nothing a suggestion reads
+  DevBuf ped_member, ped_okey, ped_work, ped_cols, ped_grid, ped_counts, ped_pdf, ped_imp, ped_loss;
 };
 
 namespace {
@@ -1779,7 +1782,9 @@ void tpe_ctx_destroy(tpe_ctx* ctx) {
                     &ctx->mo_sample, &ctx->mo_surv, &ctx->mo_nsurv, &ctx->mo_fv, &ctx->mo_ps, &ctx->mo_map, &ctx->mo_front, &ctx->mo_head,
                     &ctx->mo_contrib, &ctx->mo_state, &ctx->mo_arena, &ctx->mo_chosen, &ctx->mo_diag, &ctx->mo_w, &ctx->cols, &ctx->row_ok, &ctx->member,
                     &ctx->counts, &ctx->split_work, &ctx->below_all, &ctx->kpart, &ctx->mixcols, &ctx->ub_arena, &ctx->ub_ord_a, &ctx->ub_ord_b, &ctx->ub_wstage, &ctx->uxs, &ctx->ucidx, &ctx->uni_prev_rows, &ctx->uni_mode, &ctx->uni_work, &ctx->sort_val, &ctx->sort_idx, &ctx->sort_work, &ctx->U, &ctx->S,
-                    &ctx->xT, &ctx->x64s, &ctx->x32s, &ctx->e32s, &ctx->gmax, &ctx->lse_gmax, &ctx->mt_state, &ctx->U2, &ctx->mt_spec, &ctx->mt_jump, &ctx->mt_tmp, &ctx->oob, &ctx->logl, &ctx->logg, &ctx->out_x, &ctx->out_acq, &ctx->out_best})
+                    &ctx->xT, &ctx->x64s, &ctx->x32s, &ctx->e32s, &ctx->gmax, &ctx->lse_gmax, &ctx->mt_state, &ctx->U2, &ctx->mt_spec, &ctx->mt_jump, &ctx->mt_tmp, &ctx->oob, &ctx->logl, &ctx->logg, &ctx->out_x, &ctx->out_acq, &ctx->out_best,
+                    &ctx->ped_member, &ctx->ped_okey, &ctx->ped_work, &ctx->ped_cols, &ctx->ped_grid, &ctx->ped_counts,
+                    &ctx->ped_pdf, &ctx->ped_imp, &ctx->ped_loss})
     b->release();
   ctx->est[0].release();
   ctx->est[1].release();
@@ -3008,5 +3013,97 @@ int tpe_probe_fp64_tflops(tpe_ctx* ctx, double* tflops) {
 }
 
 const char* tpe_last_logpdf_kernel(tpe_ctx* ctx) { return ctx ? ctx->last_kernel : "none"; }
+
+int tpe_ped_anova(tpe_ctx* ctx, const tpe_ped_cfg* cfg, const int32_t* cols, int32_t n_cols, const double* grids,
+                  const int32_t* n_grid, const double* loss, double* out_importance, int64_t* out_n,
+                  int32_t* out_counts) {
+  if (!ctx) return TPE_E_INVALID;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  if (!ctx->history_set) return fail(ctx, TPE_E_STATE, "tpe_history_set must precede tpe_ped_anova");
+  if (!cfg || !cols || n_cols <= 0 || !n_grid || !out_importance || !out_n)
+    return fail(ctx, TPE_E_INVALID, "bad tpe_ped_anova arguments");
+  if (!(0.0 < cfg->target_quantile && cfg->target_quantile < cfg->region_quantile && cfg->region_quantile <= 1.0))
+    return fail(ctx, TPE_E_INVALID, "condition 0.0 < `target_quantile` < `region_quantile` <= 1.0 must be satisfied");
+  if (!(cfg->prior_weight > 0.0)) return fail(ctx, TPE_E_INVALID, "prior_weight must be positive");
+  if (cfg->min_n_top < 1) return fail(ctx, TPE_E_INVALID, "min_n_top must be positive");
+  if (cfg->n_steps < 1 || cfg->n_steps > kPedMaxSteps)
+    return fail(ctx, TPE_E_INVALID, "n_steps must be in [1, %d]", kPedMaxSteps);
+  const int P = (int)ctx->space.size();
+  std::vector<PedCol> meta((size_t)n_cols);
+  int width = 1;
+  bool numeric = false;
+  for (int j = 0; j < n_cols; ++j) {
+    const int src = cols[j];
+    if (src < 0 || src >= P) return fail(ctx, TPE_E_INVALID, "column %d out of range", src);
+    const tpe_param_desc& d = ctx->space[src];
+    const bool is_cat = d.kind == TPE_KIND_CAT;
+    if (is_cat ? n_grid[j] != d.n_choices : (n_grid[j] < 1 || n_grid[j] > cfg->n_steps))
+      return fail(ctx, TPE_E_INVALID, "column %d: %d bins (n_choices of a categorical column, 1..n_steps otherwise)",
+                  src, n_grid[j]);
+    meta[j] = PedCol{src, is_cat ? 1 : 0, d.log ? 1 : 0, n_grid[j]};
+    width = std::max(width, (int)n_grid[j]);
+    numeric = numeric || !is_cat;
+  }
+  if (numeric && !grids) return fail(ctx, TPE_E_INVALID, "numerical columns need their grids");
+  if (set_device(ctx)) return TPE_E_CUDA;
+  const int64_t N = ctx->N;
+  const int64_t nal = std::max<int64_t>(N, 1);
+  const size_t ncnt = (size_t)n_cols * 2 * width;
+  CU(ctx->ped_member.ensure((size_t)nal));
+  CU(ctx->ped_okey.ensure((size_t)nal * 8));
+  CU(ctx->ped_work.ensure(sizeof(PedWork)));
+  CU(ctx->ped_cols.ensure(sizeof(PedCol) * n_cols));
+  CU(ctx->ped_grid.ensure((size_t)n_cols * cfg->n_steps * 8));
+  CU(ctx->ped_counts.ensure(ncnt * 4));
+  CU(ctx->ped_pdf.ensure(ncnt * 8));
+  CU(ctx->ped_imp.ensure((size_t)n_cols * 8));
+  cudaStream_t st = ctx->stream;
+  CU(cudaMemsetAsync(ctx->ped_work.p, 0, sizeof(PedWork), st));
+  CU(cudaMemsetAsync(ctx->ped_counts.p, 0, ncnt * 4, st));
+  CU(cudaMemcpyAsync(ctx->ped_cols.p, meta.data(), sizeof(PedCol) * n_cols, cudaMemcpyHostToDevice, st));
+  if (numeric)
+    CU(cudaMemcpyAsync(ctx->ped_grid.p, grids, (size_t)n_cols * cfg->n_steps * 8, cudaMemcpyHostToDevice, st));
+  const double* d_loss = nullptr;
+  if (loss) {
+    CU(ctx->ped_loss.ensure((size_t)nal * 8));
+    if (N) CU(cudaMemcpyAsync(ctx->ped_loss.p, loss, (size_t)N * 8, cudaMemcpyHostToDevice, st));
+    d_loss = ctx->ped_loss.as<double>();
+  }
+  int n_i = (int)N, pall = P, nc = n_cols, mnt = cfg->min_n_top;
+  double qt = cfg->target_quantile, qr = cfg->region_quantile;
+  const double* d_X = ctx->X.as<double>();
+  const int8_t* d_cat = ctx->cat.as<int8_t>();
+  const double* d_key = ctx->key.as<double>();
+  const PedCol* d_cols = ctx->ped_cols.as<PedCol>();
+  uint8_t* d_member = ctx->ped_member.as<uint8_t>();
+  uint64_t* d_okey = ctx->ped_okey.as<uint64_t>();
+  PedWork* d_wk = ctx->ped_work.as<PedWork>();
+  void* args[] = {&n_i, &pall, &d_X, &d_cat, &d_key, &d_loss, &d_cols, &nc, &qt, &qr, &mnt, &d_member, &d_okey, &d_wk};
+  const int G = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->sm_count, (N + 1023) / 1024));
+  CU(cudaLaunchCooperativeKernel((const void*)k_ped_select_coop, dim3(G), dim3(kPedThreads), args, 0, st));
+  // histograms: shared memory unless a categorical column is too wide for it (global integer atomics then)
+  const bool use_smem = (size_t)2 * width * 4 <= 32768;
+  const size_t smem = (size_t)cfg->n_steps * 8 + (use_smem ? (size_t)2 * width * 4 : 0);
+  const int bx = (int)std::max<int64_t>(1, std::min<int64_t>((N + 4095) / 4096,
+                                                                  std::max(1, ctx->sm_count * 8 / n_cols)));
+  if (N > 0)
+    k_ped_bin<<<dim3(bx, n_cols), 256, smem, st>>>(n_i, pall, d_X, d_member, d_cols, ctx->ped_grid.as<double>(),
+                                                   cfg->n_steps, width, use_smem ? 1 : 0, ctx->ped_counts.as<int>());
+  k_ped_estimate<<<dim3(n_cols, cfg->evaluate_on_local ? 2 : 1), 128, 0, st>>>(
+      d_cols, ctx->ped_counts.as<int>(), width, d_wk, mnt, cfg->prior_weight, ctx->ped_pdf.as<double>());
+  k_ped_divergence<<<(n_cols + 127) / 128, 128, 0, st>>>(d_cols, n_cols, width, d_wk, mnt, cfg->evaluate_on_local ? 1 : 0,
+                                                         ctx->ped_pdf.as<double>(), ctx->ped_imp.as<double>());
+  CU(cudaGetLastError());
+  unsigned long long n3[3];
+  CU(cudaMemcpyAsync(n3, ctx->ped_work.p, sizeof(n3), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(out_importance, ctx->ped_imp.p, (size_t)n_cols * 8, cudaMemcpyDeviceToHost, st));
+  if (out_counts) CU(cudaMemcpyAsync(out_counts, ctx->ped_counts.p, ncnt * 4, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  const bool none = (int64_t)n3[0] <= cfg->min_n_top;
+  out_n[0] = (int64_t)n3[0];
+  out_n[1] = none ? 0 : (int64_t)n3[1];
+  out_n[2] = none ? 0 : (int64_t)n3[2];
+  return TPE_OK;
+}
 
 }  // extern "C"

@@ -361,6 +361,29 @@ class TPEEngine:
         self._check(self._lib.tpe_get_split_info(self._h, C.byref(info)))
         return int(info.n_below_all), int(info.n_below_obs), int(info.n_above_obs)
 
+    # -- importance --------------------------------------------------------------------------------
+    def ped_anova(self, cols: Sequence[int], grids, n_grid, *, target_quantile: float, region_quantile: float,
+                  evaluate_on_local: bool, loss=None, prior_weight: float = 1.0, min_n_top: int = 2,
+                  n_steps: int = 50, counts: bool = False):
+        """PED-ANOVA importance of the history columns `cols` (tpe_ped_anova).  grids [n_cols, n_steps]: the host's
+        np.linspace grid per numerical column (rows of categorical columns are ignored); n_grid [n_cols]: bins per
+        column; loss [history size] or None = the uploaded sort key.  Returns (importances [n_cols], (kept, target,
+        region), counts [n_cols, 2, max n_grid] of the target / region bins, or None)."""
+        cols_a = np.ascontiguousarray([int(c) for c in cols], dtype=np.int32)
+        ng = np.ascontiguousarray(n_grid, dtype=np.int32).reshape(-1)
+        g = _f64(grids, (len(cols_a), int(n_steps)))
+        lv = None if loss is None else _f64(loss).reshape(-1)
+        if lv is not None:
+            assert lv.size == self.history_size, (lv.size, self.history_size)
+        c = _lib.PedCfg(float(target_quantile), float(region_quantile), float(prior_weight), int(bool(evaluate_on_local)),
+                        int(min_n_top), int(n_steps))
+        imp = np.empty(len(cols_a), dtype=np.float64)
+        sizes = np.empty(3, dtype=np.int64)
+        cnt = np.empty((len(cols_a), 2, int(ng.max(initial=1))), dtype=np.int32) if counts else None
+        self._check(self._lib.tpe_ped_anova(self._h, C.byref(c), _ptr(cols_a), len(cols_a), _ptr(g), _ptr(ng), _ptr(lv),
+                                            _ptr(imp), _ptr(sizes), _ptr(cnt)))
+        return imp, tuple(int(v) for v in sizes), cnt
+
     # -- inspection --------------------------------------------------------------------------------
     def get_split(self) -> tuple[np.ndarray, np.ndarray]:
         below = np.empty(self._info[1], dtype=np.int64)
